@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the render hot path on BASELINE.json's headline workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A *step* renders one frame of each headline scene — rgbbox 1000x1000 and irreg 1000x1000 at 64 samples
@@ -200,6 +200,23 @@ def full_frame_equals_oracle(frame, key):
     return hashlib.sha256(np.ascontiguousarray(frame, "<i4").tobytes()).hexdigest() == known["sha256_le_i32"]
 
 
+DUMP_BYTES = 48 * 10**6   # all arrays --dump-outputs writes together
+
+
+def dump_outputs(out_dir, frames):
+    """--dump-outputs: every int32[h][w] frame of `frames` as out_dir/<name>.npy in float64 (exact for every int32).  When
+    the frames would take more than DUMP_BYTES, each is written as a 1-D array of its pixels at a fixed sample of row-major
+    positions (seed 0, ascending), the same positions in every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // (8 * len(frames))
+    for name, frame in frames.items():
+        out = np.asarray(frame).astype(np.float64)
+        if out.size > cap:
+            out = out.reshape(-1)[np.sort(np.random.default_rng(0).choice(out.size, cap, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), out)
+
+
 def issue_roofline(work, ms, sm_count, sm_mhz):
     """Instruction-issue roofline of a render launch: useful thread-instructions of the REFERENCE traversal's box and
     sphere tests / (SMs x 4 schedulers x 32 lanes x clock x time).  This, not HBM, is what bounds the kernel."""
@@ -221,12 +238,15 @@ def run_reference(args):
         cpu_sample()
     segs = secs = 0.0
     cores = 1
+    kept = {}
     t_all = time.perf_counter()
     for _ in range(args.steps):
-        s, t, cores = cpu_sample()
+        s, t, cores = cpu_sample(keep=kept)
         segs += s
         secs += t
     wall = time.perf_counter() - t_all
+    if args.dump_outputs:   # the last step's frames: the sampled rows, zeros elsewhere
+        dump_outputs(args.dump_outputs, kept)
     value = segs / secs / 1e6
     sample = f"rows j%{ROW_STEP}==0 of every {W}x{H} frame of the step at {SPP} spp (1/{ROW_STEP} of a step) per step"
     line = {
@@ -261,6 +281,8 @@ def run_ours(args):
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if world != args.gpus and world > 1:
         raise SystemExit(f"--gpus {args.gpus} but WORLD_SIZE={world}")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs --gpus 1")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device (the product has no CPU path; use --impl reference for the CPU arm)")
     torch.cuda.set_device(local_rank)
@@ -371,6 +393,8 @@ def run_ours(args):
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     dev_ms = float(t.item())
+    if args.dump_outputs:   # the frames of the last timed step, before the passes below render into the same buffers
+        dump_outputs(args.dump_outputs, {n: frames[n].cpu().numpy() for n in SCENES})
     value = seg_per_step * args.steps / (dev_ms * 1e-3) / 1e6
     strict = None
     if can_pipeline:   # the same K steps in the round-1 protocol, for comparison
@@ -710,6 +734,10 @@ def main():
                     help="N > 1: peer = ranks write their pixels straight into rank 0's frame over NVLink (default); nccl = tile buffers + ncclGather + de-tile")
     ap.add_argument("--workload", default="headline", choices=sorted(WORKLOADS),
                     help="headline = BASELINE configs[1]+[2] (the default the driver measures); irreg4000 = configs[3]")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the frames of the last step as DIR/<scene>.npy (float64 packed 0x00RRGGBB "
+                         "pixels, a fixed sample of them for frames beyond 48 MB in all; the scenes are fixed, so the same "
+                         "arguments give the same inputs in every run)")
     args = ap.parse_args()
     select_workload(args.workload)
     if args.impl == "reference":

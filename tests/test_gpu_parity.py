@@ -687,7 +687,7 @@ def test_single_process_multi_gpu_context(R, oracle, tmp_path):
             img2 = ctx.render(h, w, pr, spp=spp)      # buffers are reused across frames
             assert_same(img2.values(), want, f"{name} gpus={g} second frame")
             img.free(); img2.free(); pr.free()
-    exe = os.path.join(ROOT, "examples", "_built", "main_ref")
+    exe = os.path.join(ROOT, "oracle", "_ref", "main_ref")
     if os.path.exists(exe):
         ppm = str(tmp_path / "mg.ppm")
         r = subprocess.run([exe, "-s", "irreg", "-n", "120", "-m", "160", "-r", "2", "-f", ppm], capture_output=True, text=True,
@@ -700,9 +700,9 @@ def test_single_process_multi_gpu_context(R, oracle, tmp_path):
 
 
 def test_reference_driver_binary_runs_against_the_library(tmp_path, oracle):
-    """The reference's UNMODIFIED futhark/main.c, compiled in the authoring container against include/ray.h
-    (examples/_built/main_ref, see __graft_entry__.build), run here: its PPM must equal the oracle frame."""
-    exe = os.path.join(ROOT, "examples", "_built", "main_ref")
+    """The reference's UNMODIFIED futhark/main.c, compiled against include/ray.h where the original project is
+    checked out (oracle/_ref/main_ref, see __graft_entry__.build), run here: its PPM must equal the oracle frame."""
+    exe = os.path.join(ROOT, "oracle", "_ref", "main_ref")
     if not os.path.exists(exe):
         exe = os.path.join(ROOT, "examples", "_built", "driver")
     if not os.path.exists(exe):
