@@ -190,6 +190,34 @@ int ray_b200_flag_status(struct futhark_context *ctx, int64_t *timeouts);
 /* Enqueue on `stream`: device -> host copy (host_dst should be page-locked for the copy to be asynchronous). */
 int ray_b200_copy_to_host_async(struct futhark_context *ctx, void *stream, void *host_dst, const void *dev_src, int64_t bytes);
 
+/* ---- ray queries: closest hit and path colour of caller-supplied rays ----------------------------------
+ * A ray is 6 floats {origin.xyz, direction.xyz} (the layout of oracle_aabb_hit's ray6); the direction need not be
+ * normalised, just as get_ray's is not (ray.fut:109-114).  Output i always belongs to ray i.  0 <= n <= 2^30.
+ *
+ * intersect = objs_hit bvh r 0.0 1e9 (ray.fut:76-86) exactly as render uses it: boxes are tested against the original
+ *   interval, the closest-hit search uses t_min = 0.1 with strict `<`, ties go to the lowest Morton-sorted leaf, and the
+ *   winner is re-intersected with (0, t_best + 1); if that re-intersection fails the ray has no hit.  Per ray:
+ *     index[i]  int32: the hit sphere's index in the SCENE's order (the order ray_b200_scene_get_arrays returns), -1 = none
+ *     t[i]      float: hit.t of the re-intersection, +inf = none
+ *     pn[i*6]   float[6] (optional, NULL = not written): hit.p, hit.normal as sphere_hit computes them, 0 = none
+ * trace = ray_colour objs r 50 (ray.fut:126-148).  Per ray: colour[i*3] float[3], before quantisation.
+ * There are no per-ray t intervals, no depth argument and no any-hit mode: the reference defines none of them.
+ *
+ * The _into variants take device pointers and are asynchronous on the context's stream; the _host variants take host
+ * buffers and return when the results are there.  Bad arguments (n out of range, a NULL ray or required output pointer,
+ * an invalid prepared scene) return an error and launch nothing; n = 0 returns 0 and launches nothing.  A shard set with
+ * ray_b200_context_set_shard does not apply: every ray is answered.  On a single-process multi-GPU context
+ * (RAY_GPUS > 1) these calls return an error.  The prepared scene may be freed right after an asynchronous query: its
+ * device memory is released behind the query in stream order. */
+int ray_b200_intersect_into(struct futhark_context *ctx, const struct futhark_opaque_prepared_scene *p,
+                            const float *rays_dev, int64_t n, int32_t *index_dev, float *t_dev, float *pn_dev);
+int ray_b200_trace_into(struct futhark_context *ctx, const struct futhark_opaque_prepared_scene *p,
+                        const float *rays_dev, int64_t n, float *colour_dev);
+int ray_b200_intersect_host(struct futhark_context *ctx, const struct futhark_opaque_prepared_scene *p,
+                            const float *rays_host, int64_t n, int32_t *index_host, float *t_host, float *pn_host);
+int ray_b200_trace_host(struct futhark_context *ctx, const struct futhark_opaque_prepared_scene *p,
+                        const float *rays_host, int64_t n, float *colour_host);
+
 /* ---- work counters (roofline numerators) ---------------------------------------------------------- */
 struct ray_b200_counters { uint64_t segments, node_steps, box_tests, leaf_tests; };
 /* Re-renders (1 spp) with counting kernels and returns the work the GPU traversal did. */

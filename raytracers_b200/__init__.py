@@ -135,6 +135,10 @@ def load_library(variant=""):
         "ray_b200_render_into": (C.c_int, [vp, vp, vp, i64, i64, i32, vp]),
         "ray_b200_render_host": (C.c_int, [vp, vp, vp, i64, i64, i32, vp]),
         "ray_b200_entry_render_spp": (C.c_int, [vp, pp, i64, i64, i32, vp]),
+        "ray_b200_intersect_into": (C.c_int, [vp, vp, vp, i64, vp, vp, vp]),
+        "ray_b200_trace_into": (C.c_int, [vp, vp, vp, i64, vp]),
+        "ray_b200_intersect_host": (C.c_int, [vp, vp, vp, i64, vp, vp, vp]),
+        "ray_b200_trace_host": (C.c_int, [vp, vp, vp, i64, vp]),
         "ray_b200_shard_tiles": (i64, [i64, i64, i32, i32]),
         "ray_b200_shard_tiles_padded": (i64, [i64, i64, i32]),
         "ray_b200_render_shard_into": (C.c_int, [vp, vp, i64, i64, i32, vp]),
@@ -504,6 +508,40 @@ class Context:
         rgb = np.empty((h, w, 3), np.float32) if want_rgb else None
         self._check(self.lib.ray_b200_render_host(self.handle, _ptr(pix), _ptr(rgb), int(h), int(w), int(spp), prepared.handle))
         return (pix, rgb) if want_rgb else pix
+
+    def intersect_into(self, rays_dev, n, prepared, index_dev, t_dev, pn_dev=None):
+        """Closest hit of n device rays (float32[n][6]: origin, direction) into device int32[n] / float32[n] /
+        optional float32[n][6]; asynchronous on the context's stream (include/ray_b200.h "ray queries")."""
+        self._check(self.lib.ray_b200_intersect_into(self.handle, prepared.handle, _ptr(rays_dev), int(n), _ptr(index_dev),
+                                                     _ptr(t_dev), _ptr(pn_dev)))
+
+    def trace_into(self, rays_dev, n, prepared, colour_dev):
+        """Path colour (ray_colour, 50 bounces) of n device rays into device float32[n][3]; asynchronous."""
+        self._check(self.lib.ray_b200_trace_into(self.handle, prepared.handle, _ptr(rays_dev), int(n), _ptr(colour_dev)))
+
+    @staticmethod
+    def _rays(rays):
+        if not isinstance(rays, np.ndarray) or rays.dtype != np.float32 or rays.ndim != 2 or rays.shape[1] != 6:
+            raise RayError("rays must be a numpy float32 array of shape (n, 6): origin.xyz, direction.xyz")
+        return np.ascontiguousarray(rays)
+
+    def intersect(self, prepared, rays, want_pn=False):
+        """Closest hit of each ray: (index int32[n] in the scene's sphere order or -1, t float32[n] or +inf), plus
+        pn float32[n][6] (hit point, normal; 0 on a miss) when want_pn."""
+        r = self._rays(rays)
+        n = r.shape[0]
+        index = np.empty(n, np.int32)
+        t = np.empty(n, np.float32)
+        pn = np.empty((n, 6), np.float32) if want_pn else None
+        self._check(self.lib.ray_b200_intersect_host(self.handle, prepared.handle, _ptr(r), n, _ptr(index), _ptr(t), _ptr(pn)))
+        return (index, t, pn) if want_pn else (index, t)
+
+    def trace(self, prepared, rays):
+        """Colour of each ray's path (ray_colour, 50 bounces, before quantisation): float32[n][3]."""
+        r = self._rays(rays)
+        colour = np.empty((r.shape[0], 3), np.float32)
+        self._check(self.lib.ray_b200_trace_host(self.handle, prepared.handle, _ptr(r), r.shape[0], _ptr(colour)))
+        return colour
 
     def shard_tiles(self, h, w, rank, world):
         return int(self.lib.ray_b200_shard_tiles(int(h), int(w), int(rank), int(world)))
